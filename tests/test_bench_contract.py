@@ -32,5 +32,5 @@ def test_reference_arm_line(refc):
     assert "not a full encode" in d["metric_scope"]
 
 
-def test_reference_arm_other_ranks_print_nothing(refc):
+def test_reference_arm_other_ranks_print_nothing():
     assert _run({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"}) == ""

@@ -1,6 +1,7 @@
 """GPU parity at picture scale: one frame through the T2 pipeline (the path bench.py times) against
 the reference arm -- the reference's own kernels driven by oracle/ref_driver.c -- bit for bit, at a
-small size and at BASELINE's 1920x1080."""
+small size and at BASELINE's 1920x1080 (through the committed digests of tests/golden/frame_*.json where
+oracle/_ref is not built)."""
 import pytest
 
 pytestmark = pytest.mark.gpu
@@ -12,7 +13,7 @@ FRAME_CASES = [(384, 256, 8, 8), (384, 256, 10, 6), (448, 320, 10, 4), (1920, 10
 
 
 @pytest.mark.parametrize("case", FRAME_CASES, ids=lambda c: "%dx%d_b%d_m%d" % c)
-def test_frame_pipeline_matches_reference(b200, refc, case):
+def test_frame_pipeline_matches_reference(b200, case):
     """every output of the T2 frame pipeline == the reference's own kernels (8-bit: svt_av1_inv_txfm_add, svt_av1_compute_stats,
     svt_av1_wiener_convolve_add_src ...; 10-bit: svt_aom_inv_transform_recon with CONVERT_TO_BYTEPTR planes as in
     full_loop.c:1843-1846, svt_av1_highbd_quantize_fp_qm, svt_compute_cdef_dist_16bit, svt_av1_compute_stats_highbd,
@@ -31,7 +32,7 @@ def test_frame_pipeline_matches_reference(b200, refc, case):
     assert torch.equal(a[0], fp.final) and torch.equal(a[1], fp.qcoeff) and torch.equal(a[2], fp.me["me_mv_array"])
 
 
-def test_cdef_apply_recomputes_directions_when_none_given(b200, refc):
+def test_cdef_apply_recomputes_directions_when_none_given(b200):
     """svt_b200_cdef_apply_frame_dev with d_dir = d_var = NULL finds the directions itself; the result
     must equal the apply that reuses the arrays of the search."""
     import ctypes as ct
@@ -57,7 +58,7 @@ def test_cdef_apply_recomputes_directions_when_none_given(b200, refc):
                                                  fp.app_uv.data_ptr(), fp.cdef_dir.data_ptr(), None, oy, ocb, ocr, sy, sc, s) == -4  # SVT_B200_ERR_BAD_ARG
 
 
-def test_two_frames_in_flight_on_two_streams(b200, refc):
+def test_two_frames_in_flight_on_two_streams(b200):
     """bench.py keeps two independent frames in flight on two streams (CUDA-graph replays); every library
     scratch buffer is per stream, so the concurrent results must equal the one-at-a-time results."""
     import torch
@@ -103,7 +104,7 @@ def test_two_frames_in_flight_on_two_streams(b200, refc):
 @pytest.mark.parametrize("name", ["frame_384x256", "frame_640x360", "frame_384x256_b10_m6", "frame_640x360_b10_m4"])
 def test_frame_matches_committed_golden_fixture(b200, name):
     """tests/golden/frame_WxH.json holds the SHA-256 of every output of the frame as computed by the reference's
-    own C kernels (tools/make_golden.py, run where /root/reference exists).  Needs no oracle at run time."""
+    own C kernels (tools/make_golden.py, run where oracle/_ref is built).  Needs no oracle at run time."""
     import hashlib
     import json
     import os

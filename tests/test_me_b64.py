@@ -44,10 +44,12 @@ CASES = [
 
 
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
-def test_me_b64_matches_reference_driver(b200, refc, case):
+def test_me_b64_matches_reference_driver(b200, oracle, golden, case):
     import torch
     name, W, H, preset, n_ref, dist, tl, is_ref, extra, content = case
-    refc.ref_set_tier(0)
+    refc = oracle.ref
+    if refc is not None:
+        refc.ref_set_tier(0)
     r = rng(500 + len(name))
     shapes = b200.me_plane_shapes(W, H)
     n_pic = n_ref[0] + n_ref[1] + 1
@@ -59,8 +61,9 @@ def test_me_b64_matches_reference_driver(b200, refc, case):
     cur_np = mh.build_pyramid_np(seq[mid], W, H, shapes)
     refs_np = [mh.build_pyramid_np(f, W, H, shapes) for f in fulls]
     cfg = sp.me_b64_cfg(preset=preset, n_ref=n_ref, poc_dist=dist, temporal_layer_index=tl, is_ref=is_ref, **extra)
-    ctrl, want = sp.ref_me_b64_picture(refc, cur_np, refs_np, shapes, cfg)
-    cd = ctrl.as_dict()
+    ctrl, want = sp.ref_me_b64_picture(refc, cur_np, refs_np, shapes, cfg) if refc is not None else (None, None)
+    cd = golden.value(lambda: ctrl.as_dict())  # the controls the reference derived (svt_aom_sig_deriv_me)
+    ref = (lambda k: want[k]) if want is not None else (lambda k: None)  # noqa: E731
     assert n_pic == len(fulls) + 1
 
     def upload(planes_np):
@@ -88,23 +91,23 @@ def test_me_b64_matches_reference_driver(b200, refc, case):
     torch.cuda.synchronize()
     got = {k: v.cpu().numpy() for k, v in dev.items()}
     # intermediate state first (a mismatch there explains everything after it)
-    assert np.array_equal(got["zz_sad"].view(np.uint32), want["zz_sad"]), name
-    assert np.array_equal(got["hme_centre"], want["hme_centre"]), name
-    assert np.array_equal(got["do_ref"], want["do_ref"]), name
+    golden.check(got["zz_sad"].view(np.uint32), ref("zz_sad"), name)
+    golden.check(got["hme_centre"], ref("hme_centre"), name)
+    golden.check(got["do_ref"], ref("do_ref"), name)
     k = 0
     for li in range(2):
         for ri in range(n_ref[li]):
-            live = want["do_ref"][:, li, ri].astype(bool)
+            live = got["do_ref"][:, li, ri].astype(bool)
             # references pruned after the full-pel search (me_prune_ref) still hold their search results in both; earlier-pruned ones are undefined
-            assert np.array_equal(got["best_sad"][k].view(np.uint32)[live], want["best_sad"][:, li, ri][live]), (name, li, ri)
-            assert np.array_equal(got["best_mv"][k].view(np.uint32)[live], want["best_mv"][:, li, ri][live]), (name, li, ri)
+            golden.check(got["best_sad"][k].view(np.uint32)[live], want and want["best_sad"][:, li, ri][live], name, li, ri)
+            golden.check(got["best_mv"][k].view(np.uint32)[live], want and want["best_mv"][:, li, ri][live], name, li, ri)
             k += 1
     # what the rest of the encoder consumes
-    for key in ("total_me_candidate_index", "me_candidate_array", "distortion", "flags"):
-        assert np.array_equal(got[key].view(want[key].dtype), want[key]), (name, key)
-    assert np.array_equal(got["me_mv_array"].view(np.uint32), want["me_mv_array"]), name
+    for key, dt in (("total_me_candidate_index", np.uint8), ("me_candidate_array", np.uint8), ("distortion", np.uint32), ("flags", np.uint8)):
+        golden.check(got[key].view(dt), ref(key), name, key)
+    golden.check(got["me_mv_array"].view(np.uint32), ref("me_mv_array"), name)
     # the case must exercise what it is there for
     if name == "m8_nonbase_2p2":
-        assert (want["do_ref"][:, :, 1] == 0).any() and (want["zz_sad"][:, 0, 0] < cd["me_early_exit_th"]).any()
+        assert (got["do_ref"][:, :, 1] == 0).any() and (got["zz_sad"].view(np.uint32)[:, 0, 0] < cd["me_early_exit_th"]).any()
     if name == "m4_mrp_off_gm":
-        assert want["flags"][:, 1].any()
+        assert got["flags"][:, 1].any()

@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Generate tests/golden/frame_<W>x<H>.json: SHA-256 of every output of one synthetic frame computed by the
-REFERENCE's own kernels (oracle/_ref, C tier, driven by oracle/ref_driver.c).  Run in the build container (where
-/root/reference exists and `python __graft_entry__.py --oracle` has built oracle/_ref); the fixture travels with
-the repository so that the GPU parity test also works where oracle/_ref is absent."""
+REFERENCE's own kernels (oracle/_ref, C tier, driven by oracle/ref_driver.c).  Run where `python __graft_entry__.py --oracle`
+has built oracle/_ref (it needs the reference source tree); the fixtures are committed so that the GPU parity tests and
+smoke() also work where oracle/_ref is absent.  One fixture per picture size of test_frame_pipeline.FRAME_CASES."""
 import hashlib
 import json
 import os
@@ -37,7 +37,8 @@ def golden_for(width, height, seed=20260923, bit_depth=8, preset=8):
 
 
 if __name__ == "__main__":
-    for (w, h, bd, m) in ((384, 256, 8, 8), (640, 360, 8, 8), (384, 256, 10, 6), (640, 360, 10, 4)):
+    for (w, h, bd, m) in ((384, 256, 8, 8), (640, 360, 8, 8), (384, 256, 10, 6), (640, 360, 10, 4), (448, 320, 10, 4), (1920, 1080, 8, 8),
+                          (1920, 1080, 10, 6), (3840, 2160, 8, 8), (3840, 2160, 10, 4)):
         g = golden_for(w, h, bit_depth=bd, preset=m)
         path = os.path.join(ROOT, "tests", "golden", "frame_%dx%d%s.json" % (w, h, "" if (bd, m) == (8, 8) else "_b%d_m%d" % (bd, m)))
         json.dump(g, open(path, "w"), indent=1, sort_keys=True)
