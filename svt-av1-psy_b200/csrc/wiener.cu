@@ -10,12 +10,10 @@
 //     M[k] += y[k] x, H[k][l] += y[k] y[l]; high bit depth divides by 4 / 16 at the end (truncating).
 //
 // B200 mapping of the statistics (the one dense contraction on the path):
-//   8-bit pixels -> stats_mma_kernel: exact f16 x f16 -> f32 tensor-core MMA (see the comment above it);
+//   8-bit pixels -> stats_mma_kernel: exact u8 x u8 -> s32 tcgen05 MMA on the raw pixels (see the comment above it);
 //   10/12-bit    -> the lag-sum kernels of wiener_stats_lag.cuh (H[p][q] depends only on the lag between the two samples).
-// The MMA kernel writes per-CTA int64 partials; stats_finalize_kernel adds them, mirrors the triangle and applies
-// the bit-depth divider.
-#include <cuda_fp16.h>
-
+// The MMA kernel writes per-CTA int64 partials; stats_finalize_kernel adds them, folds the mean back in and mirrors
+// the triangle.
 #include <map>
 
 #include "common.cuh"
@@ -79,242 +77,347 @@ stats_sum_kernel(const PIX* __restrict__ dgd_base, const SvtB200StatsItem* __res
     if (lane == 0 && wide) atomicAdd(&tot_out[it], wide);
 }
 
-__device__ __forceinline__ int stats_average(const unsigned long long* tot, int it, const SvtB200StatsItem& s) {
-    return (int)(tot[it] / (unsigned long long)((s.h_end - s.h_start) * (s.v_end - s.v_start)));
-}
-
 constexpr int kStatsMaxParts = 32;  // CTAs cooperating on one restoration unit
 
-// partial layout per (item, part): [0, 49*49) = H (upper-triangle tiles only), [2401, 2450) = M
-//
-
 // ---------------------------------------------------------------------------------------------
-// K11, 8-bit pixels: the contraction on the tensor cores.
+// K11, 8-bit pixels: the contraction on the tensor cores (tcgen05.mma, kind::i8).
 //
-// H = Y^T Y is a Gram matrix with K = pixels.  |pixel - avg| <= 255 is exact in f16, every product
-// (<= 255^2) is exact in f32 and a sum of up to 256 of them stays below 2^24, so an f16 x f16 -> f32
-// MMA chain over 256 pixels is EXACT integer arithmetic; the f32 accumulators are then converted and
-// added to int32 totals in shared memory (good for 33025 pixels), which fold into the CTA's int64
-// partial.  Bit-exact with the reference for any input; tests/test_wiener.py holds the extremes.
+// The MMA runs on the RAW pixels (dgd - avg does not fit in 8 bits).  With G the Gram matrix of the raw window vectors,
+// S_k the sum of window sample k over the region, Sx the source sum and n the pixel count, the reference's sums are
+//   H_kl = G_kl - v (S_k + S_l) + n v^2,   M_k = G_kx - v S_k - v Sx + n v^2,   v = avg = S_centre / n
+// (S_centre is the sum find_average divides by n), evaluated in int64 by stats_finalize_kernel.  u8 x u8 products
+// (<= 255^2) accumulate in s32 tensor memory, exact for kTcFoldPixels pixels; past that the CTA folds TMEM into its
+// int64 partial.  Bit-exact with the reference for any input; tests/test_wiener.py holds the extremes.
 //
-// Matrix rows are ordered i = 8*kx + ky (window column kx, window row ky < WIN); row 7 is x = src - avg
-// (so M = row 7 of the same product) and rows with ky >= WIN are don't-care padding.  One
-// mma.m16n8k16 K-step covers a 2-row x 8-column block of pixels, k = 2*column + row: a fragment
-// register then holds (d[r][c], d[r+1][c]), which the tile stores pre-paired as one 32-bit word per
-// (r, c) -- any window shift is a plain word index, and with a row pitch == 4 (mod 32) words the 8
-// window rows x 4 columns a warp fetches per load land in 32 distinct banks.  The B fragment of
-// n-tile kx is also one half of the A fragment of m-tile kx/2, so a K-step costs 2*WIN loads for
-// all of its MMAs.  Only the tiles of the upper triangle (m-tile m, n-tile n >= 2m) are computed.
-constexpr int kMmaWarps = 4;
-constexpr int kMmaTW = 64, kMmaTH = 32;
-constexpr int kMmaPitch = 100;                                // words per pair-row
-constexpr int kMmaPRows = kMmaTH + 8;                         // py <= TH-2, plus window/padding row <= 8
-constexpr int kMmaXBase = kMmaPRows * kMmaPitch + 28;         // x rows sit on banks 28..31 like a window row 7
-constexpr int kMmaWords = kMmaXBase + kMmaTH * kMmaPitch;
-constexpr int kMmaAccMax = 16 * 128;                          // 16 output tiles x 128 accumulators (WIN = 7)
-constexpr int kMmaFoldPixels = 33025 - kMmaTW * kMmaTH;       // 2^31 / 255^2, minus the tile about to be added
-static_assert(kMmaPitch % 32 == 4 && (kMmaPRows * kMmaPitch) % 32 == 0, "bank layout");
-static_assert(kMmaTW + 6 <= kMmaPitch && kMmaAccMax <= 2450, "layout");
-
-__device__ __forceinline__ void mma_16816_f16f32(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
-                                                 uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};\n"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+// Operand (K = pixels, 32 per MMA; a tile = up to kTcTW pixels of stats_tile_rows(WIN) rows): for every image row r of
+// the tile (tile rows -WIN/2 .. last + WIN/2) the CTA writes one 8-row GROUP: row dx < WIN is dgd row r shifted by
+// dx - WIN/2, row 7 is src row r; columns past the region's width are zero in every row.  Layout: K-major, no swizzle,
+// 16-byte core-matrix rows, LBO = 128 B along K, SBO = kTcGrpBytes between groups.  One descriptor starting at the group
+// of row y - WIN/2 is both A and B of an M = N = 128 MMA (16 groups), so with a = 8 dy + dx
+//   D[a + 8t][b + 8t] = sum over the MMA's 32 pixels of output row y + t of  (window sample a) * (window sample b):
+// the window products of T = stats_block_rows(WIN) consecutive output rows at once, on the 8-row diagonals of D
+// (column b = 8 (WIN/2) + 7 is the source sample: G_kx).  A tile issues one MMA per block of T rows and 32 pixels; the
+// readback sums G(a, b) = sum_t D[a + 8t][b + 8t].  D row i is TMEM lane i (PTX ISA data-path layout for M = 128,
+// cta_group::1); the entries off those diagonals are don't-care.  Blocks run into a D at TMEM column 0; the short last
+// block of a region's bottom tiles runs into a second D at column 128 whose diagonals are summed over its own row count.
+// S_k and Sx come from per-(group, row) byte sums (DP4A) taken while the groups are written.
+//
+// One elected thread issues the MMAs of a tile and commits them to the buffer's mbarrier; the other threads build
+// the next tile into the second buffer meanwhile.
+constexpr int kTcThreads = 128;
+constexpr int kTcTW = 128;                                 // pixels per tile row (4 K-steps)
+// output rows whose window products one M = N = 128 MMA holds (a + 8t < 128 for every needed a = 8 dy + dx: 10, 12, 14),
+// and the rows of a tile: a whole number of blocks, at most 36
+__host__ __device__ constexpr int stats_block_rows(int win) { return (127 - 9 * (win - 1)) / 8 + 1; }
+__host__ __device__ constexpr int stats_tile_rows(int win) { return stats_block_rows(win) * (36 / stats_block_rows(win)); }
+constexpr int kTcGrpBytes = 8 * 128 + 16;                  // +16: the 8 groups a quarter warp writes land on distinct banks
+constexpr int kTcGroups = 40;                              // every WIN: >= rows + WIN - 1 written, >= rows - T + 16 read
+constexpr int kTcBufBytes = kTcGroups * kTcGrpBytes;
+constexpr int kTcRowSums = kTcGroups * 8;                  // byte sum of every (group, row) of a tile
+constexpr int kTcDumpPitch = 129;                          // words per D row when D is read back through shared memory
+constexpr int kTcSmem = 2 * kTcBufBytes + 2 * kTcRowSums * 4 + 32;
+constexpr int kTcFoldPixels = 33025;                       // 2^31 / 255^2: the s32 accumulators stay exact
+constexpr int kTcTmemCols = 256;                           // two 128-column D
+constexpr bool stats_tc_fits(int win) {
+    return stats_tile_rows(win) + win - 1 <= kTcGroups && stats_tile_rows(win) - stats_block_rows(win) + 16 <= kTcGroups;
 }
+static_assert(stats_tc_fits(7) && stats_tc_fits(5) && stats_tc_fits(3), "operand buffer");
+static_assert(128 * kTcDumpPitch * 4 <= 2 * kTcBufBytes, "D is read back through the operand buffers");
+static_assert(kTcBufBytes % 16 == 0 && kTcSmem < 227 * 1024 / 2, "two CTAs per SM (2 x 256 TMEM columns)");
 
-// (lo, hi), |v| <= 255, as two f16 in one word without integer->float conversions: 0x6400 + n is the
-// f16 encoding of 1024 + n for 0 <= n < 1024, and subtracting 1280 from 1024 + (v + 256) is exact.
-__device__ __forceinline__ uint32_t pack_pair_f16(int lo, int hi) {
-    const uint32_t bits = 0x64006400u + (uint32_t)(lo + 256) + ((uint32_t)(hi + 256) << 16);
-    const __half2  h    = __hsub2(*reinterpret_cast<const __half2*>(&bits), __float2half2_rn(1280.f));
-    return *reinterpret_cast<const uint32_t*>(&h);
-}
+// per-CTA partial (int64 words): the upper triangle of G by reference index (row p holds columns q >= p), G_kx, S_k, Sx
+// and n -- everything exact, combined and expanded by stats_finalize_kernel
+constexpr int kPartG = 0, kPartGx = 1225, kPartS = kPartGx + 49, kPartSx = kPartS + 49, kPartN = kPartSx + 1;
+constexpr int kStatsPartWords = kPartN + 1;
+constexpr size_t kStatsItemWords = (size_t)kStatsMaxParts * kStatsPartWords;  // scratch words per item (either path)
+static_assert(kStatsItemWords >= (size_t)kLagItemWords, "the lag path shares the scratch");
 
-__host__ __device__ __forceinline__ int mma_tile_index(int win, int m, int n) { return m * win - m * (m - 1) + n - 2 * m; }
+__host__ __device__ __forceinline__ int stats_tri_index(int w2, int p, int q) { return p * w2 - p * (p - 1) / 2 + q - p; }
 // CTAs of an item that actually get pixel tiles (and so write a partial)
 __device__ __forceinline__ int stats_mma_parts(const SvtB200StatsItem& s, int ctas_per_item) {
-    const int tiles = ((s.h_end - s.h_start + kMmaTW - 1) / kMmaTW) * ((s.v_end - s.v_start + kMmaTH - 1) / kMmaTH);
+    const int th = stats_tile_rows(s.wiener_win);
+    const int tiles = ((s.h_end - s.h_start + kTcTW - 1) / kTcTW) * ((s.v_end - s.v_start + th - 1) / th);
     return tiles < ctas_per_item ? tiles : ctas_per_item;
 }
 
-template <int WIN>
-__device__ __forceinline__ void stats_mma_body(const uint8_t* __restrict__ dgd, const uint8_t* __restrict__ src, const SvtB200StatsItem& s,
-                                               const int avg, const int part, const int parts, long long* __restrict__ P,
-                                               uint32_t* __restrict__ tile, int* __restrict__ s32) {
-    constexpr int NT = WIN, MT = (WIN + 1) / 2, HALF = WIN / 2, OFF = 3 - HALF;
-    constexpr int NTILES = MT * WIN - MT * (MT - 1);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
-    // word offset of this lane's fragment row in n-tile n, relative to the K-step's (py, px) word
-    int boff[NT];
-#pragma unroll
-    for (int n = 0; n < NT; n++) boff[n] = (OFF + g) * kMmaPitch + OFF + n + t;
-    if (g == 7) boff[0] = kMmaXBase + t;
-    float acc[NTILES][4];
-#pragma unroll
-    for (int i = 0; i < NTILES; i++) acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.f;
-    for (int i = threadIdx.x; i < NTILES * 128; i += kMmaWarps * 32) s32[i] = 0;
-    __syncthreads();
-    auto flush_regs = [&]() {
-#pragma unroll
-        for (int i = 0; i < NTILES; i++)
-#pragma unroll
-            for (int r = 0; r < 4; r++) {
-                atomicAdd(&s32[(i * 4 + r) * 32 + lane], __float2int_rn(acc[i][r]));
-                acc[i][r] = 0.f;
-            }
-    };
-    const int W = s.h_end - s.h_start, H = s.v_end - s.v_start;
-    const int ntx = (W + kMmaTW - 1) / kMmaTW, nty = (H + kMmaTH - 1) / kMmaTH;
-    const int vlo = s.v_start - HALF, vhi = s.v_end + HALF, hlo = s.h_start - HALF, hhi = s.h_end + HALF;
-    int  ksteps = 0, pending = 0;
-    bool spilled = false;
-    // pull the rows a tile needs towards L1 (one 128-byte line per request; every address is inside the
-    // region the reference itself reads): issued for tile k+1 right before the MMA loop of tile k
-    auto prefetch_tile = [&](int tl) {
-        const int ty = tl / ntx, tx = tl - ty * ntx;
-        const int r0 = s.v_start + ty * kMmaTH, c0 = s.h_start + tx * kMmaTW;
-        for (int w = threadIdx.x; w < 2 * (kMmaPRows + 1) + kMmaTH; w += kMmaWarps * 32) {
-            const uint8_t* p;
-            if (w < 2 * (kMmaPRows + 1)) {
-                const int row = min(max(r0 - 3 + (w >> 1), vlo), vhi - 1);
-                const int col = (w & 1) ? min(c0 + kMmaTW + 2, hhi - 1) : max(c0 - 3, hlo);
-                p = dgd + (ptrdiff_t)row * s.dgd_stride + col;
-            } else {
-                const int row = min(r0 + (w - 2 * (kMmaPRows + 1)), s.v_end - 1);
-                p = src + (ptrdiff_t)row * s.src_stride + min(c0 + 32, s.h_end - 1);
-            }
-            asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
-        }
-    };
-    for (int tl = part; tl < ntx * nty; tl += parts) {
-        const int ty = tl / ntx, tx = tl - ty * ntx;
-        const int r0 = s.v_start + ty * kMmaTH, c0 = s.h_start + tx * kMmaTW;
-        const int nrows = min(kMmaTH, s.v_end - r0), ncols = min(kMmaTW, s.h_end - c0);
-        if (pending > kMmaFoldPixels) {  // CTA-uniform: fold the int32 totals into the int64 partial
-            flush_regs();
-            ksteps = 0;
-            __syncthreads();
-            for (int i = threadIdx.x; i < NTILES * 128; i += kMmaWarps * 32) {
-                P[i] = (spilled ? P[i] : 0) + s32[i];
-                s32[i] = 0;
-            }
-            spilled = true;
-            pending = 0;
-        }
-        __syncthreads();
-        // pair words of d = dgd - avg for tile rows/cols -3.. (zero outside what the reference reads)
-        for (int w = threadIdx.x; w < (kMmaTW + 6) * 4; w += kMmaWarps * 32) {
-            const int  seg = w / (kMmaTW + 6), c = w - seg * (kMmaTW + 6);
-            const int  col = c0 - 3 + c;
-            const bool cv = col >= hlo && col < hhi;
-            const int  rbeg = seg * (kMmaPRows / 4);
-            auto ld = [&](int rr) {
-                const int row = r0 - 3 + rr;
-                return (cv && row >= vlo && row < vhi) ? (int)dgd[(ptrdiff_t)row * s.dgd_stride + col] - avg : 0;
-            };
-            int lo = ld(rbeg);
-#pragma unroll
-            for (int k = 0; k < kMmaPRows / 4; k++) {
-                const int hi = ld(rbeg + k + 1);
-                tile[(rbeg + k) * kMmaPitch + c] = pack_pair_f16(lo, hi);
-                lo = hi;
-            }
-        }
-        for (int w = threadIdx.x; w < (kMmaTH / 2) * kMmaTW; w += kMmaWarps * 32) {
-            const int  r = (w / kMmaTW) * 2, c = w % kMmaTW;
-            const bool cv = c < ncols;
-            const uint8_t* p = src + (ptrdiff_t)(r0 + r) * s.src_stride + c0 + c;
-            const int lo = (cv && r < nrows) ? (int)p[0] - avg : 0;
-            const int hi = (cv && r + 1 < nrows) ? (int)p[s.src_stride] - avg : 0;
-            tile[kMmaXBase + r * kMmaPitch + c] = pack_pair_f16(lo, hi);
-        }
-        __syncthreads();
-        if (tl + parts < ntx * nty) prefetch_tile(tl + parts);
-        const int cgs = (ncols + 7) >> 3, nsteps = cgs * ((nrows + 1) >> 1);
-        for (int st = warp; st < nsteps; st += kMmaWarps) {
-            const int rp = st / cgs, px = (st - rp * cgs) * 8, py = rp * 2;
-            const uint32_t* base = tile + py * kMmaPitch + px;
-            // pixels of this K-step outside the region contribute nothing: zero them in the B operand
-            const uint32_t rowmask = (py + 1 < nrows) ? 0xffffffffu : 0x0000ffffu;
-            const uint32_t m0 = (px + t < ncols) ? rowmask : 0u, m1 = (px + t + 4 < ncols) ? rowmask : 0u;
-            uint32_t f0[NT], f1[NT];
-#pragma unroll
-            for (int n = 0; n < NT; n++) {
-                f0[n] = base[boff[n]];
-                f1[n] = base[boff[n] + 4];
-            }
-#pragma unroll
-            for (int m = 0; m < MT; m++) {
-                constexpr int last = NT - 1;
-                const int     lo = 2 * m, hi = 2 * m + 1 <= last ? 2 * m + 1 : last;
-#pragma unroll
-                for (int n = 2 * m; n < NT; n++)
-                    mma_16816_f16f32(acc[m * WIN - m * (m - 1) + n - 2 * m], f0[lo], f0[hi], f1[lo], f1[hi], f0[n] & m0, f1[n] & m1);
-            }
-            if (++ksteps == 16) {  // 256 pixels: the f32 sums are still exact integers
-                flush_regs();
-                ksteps = 0;
-            }
-        }
-        pending += nrows * ncols;
-    }
-    flush_regs();
-    __syncthreads();
-    for (int i = threadIdx.x; i < NTILES * 128; i += kMmaWarps * 32) P[i] = (spilled ? P[i] : 0) + s32[i];
+__device__ __forceinline__ uint32_t tc_smem(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_bar_wait(uint64_t* bar, uint32_t parity) {
+    uint32_t ok;
+    do {
+        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                     : "=r"(ok) : "r"(tc_smem(bar)), "r"(parity) : "memory");
+    } while (!ok);
+}
+// shared-memory matrix descriptor: start >> 4, LBO = 128 B, SBO = kTcGrpBytes, descriptor version 1 (bit 46), no swizzle
+__device__ __forceinline__ uint64_t tc_desc(uint32_t addr) {
+    return (uint64_t)((addr >> 4) & 0x3fffu) | ((uint64_t)(128 >> 4) << 16) | ((uint64_t)(kTcGrpBytes >> 4) << 32) | (1ull << 46);
+}
+// instruction descriptor of kind::i8: D s32 (bits 4-5 = 2), A and B unsigned (bits 7-9, 10-12 = 0), both K-major,
+// N >> 3 at bit 17, M >> 4 at bit 24
+template <int N>
+__host__ __device__ constexpr uint32_t tc_idesc() { return (2u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24); }
+__device__ __forceinline__ void tc_mma_i8(uint32_t tmem, uint64_t desc, uint32_t idesc, uint32_t accum) {
+    asm volatile("{ .reg .pred p; setp.ne.b32 p, %3, 0;\n\t"
+                 "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %1, %2, p; }"
+                 ::"r"(tmem), "l"(desc), "r"(idesc), "r"(accum) : "memory");
+}
+__device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t (&v)[16]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
+                   "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+                 : "r"(taddr) : "memory");
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-__global__ void __launch_bounds__(kMmaWarps * 32)
+// Writes the groups of one tile into `op` and adds their per-(group, row) byte sums to `rs` (zeroed).  Only the
+// 16-byte chunks of the K-steps that will be issued are written; a chunk past the region's width is written as zeros.
+template <int WIN>
+__device__ __forceinline__ void tc_build(uint8_t* __restrict__ op, int* __restrict__ rs, const uint8_t* __restrict__ dgd,
+                                         const uint8_t* __restrict__ src, int dgd_stride, int src_stride, int r0, int c0, int nrows,
+                                         int ncols) {
+    constexpr int HALF = WIN / 2;
+    constexpr uint32_t ONES = 0x01010101u;
+    const int ng = nrows + WIN - 1, nkc = ((ncols + 31) >> 5) * 2;
+    for (int c = threadIdx.x; c < ng * nkc; c += kTcThreads) {
+        const int kc = c / ng, g = c - kc * ng;            // a quarter warp: 8 consecutive groups, one chunk
+        const int kv = min(max(ncols - 16 * kc, 0), 16);   // columns of the region in this chunk
+        uint32_t mask[4];
+#pragma unroll
+        for (int m = 0; m < 4; m++) {
+            const int vb = min(max(kv - 4 * m, 0), 4);
+            mask[m] = vb == 4 ? 0xffffffffu : (1u << (8 * vb)) - 1u;
+        }
+        uint8_t* dst = op + g * kTcGrpBytes + kc * 128;
+        int*     rsg = rs + g * 8;
+        const int r = r0 - HALF + g;
+        // dgd bytes [a, a + kv + WIN - 1) with a = column c0 - HALF + 16 kc: the aligned words holding one of them
+        const uint8_t*  p   = dgd + (ptrdiff_t)r * dgd_stride + (c0 - HALF + 16 * kc);
+        const uint32_t  off = (uint32_t)(uintptr_t)p & 3u;
+        const uint32_t* wp  = reinterpret_cast<const uint32_t*>(p - off);
+        const int       nw  = kv ? (int)(off + kv + WIN + 2) >> 2 : 0;
+        uint32_t w[7], u[6];
+#pragma unroll
+        for (int i = 0; i < 7; i++) w[i] = i < nw ? __ldg(wp + i) : 0u;
+#pragma unroll
+        for (int i = 0; i < 6; i++) u[i] = __funnelshift_r(w[i], w[i + 1], off * 8);  // bytes a + 4i ..
+#pragma unroll
+        for (int dx = 0; dx < WIN; dx++) {
+            uint32_t o[4];
+#pragma unroll
+            for (int m = 0; m < 4; m++) o[m] = __funnelshift_r(u[(dx >> 2) + m], u[(dx >> 2) + m + 1], (dx & 3) * 8) & mask[m];
+            *reinterpret_cast<uint4*>(dst + dx * 16) = make_uint4(o[0], o[1], o[2], o[3]);
+            const uint32_t sum = __dp4a(o[0], ONES, __dp4a(o[1], ONES, __dp4a(o[2], ONES, __dp4a(o[3], ONES, 0u))));
+            if (sum) atomicAdd(&rsg[dx], (int)sum);
+        }
+        if (g >= HALF && g < HALF + nrows) {  // row 7: the source row (only the tile's own rows are ever used)
+            const uint8_t*  q    = src + (ptrdiff_t)r * src_stride + c0 + 16 * kc;
+            const uint32_t  off2 = (uint32_t)(uintptr_t)q & 3u;
+            const uint32_t* wq   = reinterpret_cast<const uint32_t*>(q - off2);
+            const int       nw2  = kv ? (int)(off2 + kv + 3) >> 2 : 0;
+            uint32_t x[5], o[4];
+#pragma unroll
+            for (int i = 0; i < 5; i++) x[i] = i < nw2 ? __ldg(wq + i) : 0u;
+#pragma unroll
+            for (int m = 0; m < 4; m++) o[m] = __funnelshift_r(x[m], x[m + 1], off2 * 8) & mask[m];
+            *reinterpret_cast<uint4*>(dst + 7 * 16) = make_uint4(o[0], o[1], o[2], o[3]);
+            const uint32_t sum = __dp4a(o[0], ONES, __dp4a(o[1], ONES, __dp4a(o[2], ONES, __dp4a(o[3], ONES, 0u))));
+            if (sum) atomicAdd(&rsg[7], (int)sum);
+        }
+    }
+}
+
+template <int WIN>
+__device__ __forceinline__ void stats_tc_body(const uint8_t* __restrict__ dgd, const uint8_t* __restrict__ src, const SvtB200StatsItem& s,
+                                              const int part, const int parts, long long* __restrict__ P, uint8_t* smem) {
+    constexpr int HALF = WIN / 2, W2 = WIN * WIN, T = stats_block_rows(WIN), TH = stats_tile_rows(WIN);
+    constexpr uint32_t IDESC = tc_idesc<128>();
+    // the S loop below reads row sums up to group TH - 1 + WIN - 1, row 7 (window rows dy < WIN; Sx: dy = WIN/2, row 7)
+    static_assert((TH - 1 + WIN - 1) * 8 + 7 < kTcRowSums, "row sums of a tile");
+    int*      rsum  = reinterpret_cast<int*>(smem + 2 * kTcBufBytes);  // [2][kTcRowSums]
+    uint64_t* bar   = reinterpret_cast<uint64_t*>(rsum + 2 * kTcRowSums);
+    uint32_t* tslot = reinterpret_cast<uint32_t*>(bar + 2);
+    const int tid = threadIdx.x, warp = tid >> 5;
+    if (tid == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(tc_smem(&bar[0])) : "memory");
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(tc_smem(&bar[1])) : "memory");
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    for (int i = tid; i < 2 * kTcRowSums; i += kTcThreads) rsum[i] = 0;
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc_smem(tslot)), "r"(kTcTmemCols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = *tslot;
+
+    const int W = s.h_end - s.h_start, H = s.v_end - s.v_start;
+    const int ntx = (W + kTcTW - 1) / kTcTW, nty = (H + TH - 1) / TH, ntiles = ntx * nty;
+    const int rlast = (H - (nty - 1) * TH) % T;  // rows of the short last block of the bottom tiles (0: none)
+    // D (128 x 128 s32 at TMEM column col) -> shared memory (over the operand buffers), then the partial's G and G_kx
+    // entries (+)= sum over t < nt of D[a + 8t][b + 8t].  Every thread; the tensor core has finished.
+    auto drain_one = [&](uint32_t col, int nt, bool add) {
+        int* d = reinterpret_cast<int*>(smem);
+#pragma unroll 1
+        for (int c = 0; c < 128; c += 16) {
+            uint32_t v[16];
+            tc_ld16(tmem + ((uint32_t)(warp * 32) << 16) + col + (uint32_t)c, v);
+#pragma unroll
+            for (int j = 0; j < 16; j++) d[tid * kTcDumpPitch + c + j] = (int)v[j];
+        }
+        __syncthreads();
+        for (int e = tid; e < W2 * W2 + W2; e += kTcThreads) {
+            int p, b;
+            long long* dst;
+            if (e < W2 * W2) {
+                p = e / W2;
+                const int q = e - p * W2;
+                if (q < p) continue;
+                b   = 8 * (q % WIN) + q / WIN;  // reference index q = dx * WIN + dy -> D index 8 dy + dx
+                dst = P + kPartG + stats_tri_index(W2, p, q);
+            } else {
+                p   = e - W2 * W2;
+                b   = 8 * HALF + 7;
+                dst = P + kPartGx + p;
+            }
+            const int  a = 8 * (p % WIN) + p / WIN;
+            long long  g = 0;
+            const int* dd = d + a * kTcDumpPitch + b;
+            for (int t = 0; t < nt; t++) g += dd[t * (8 * kTcDumpPitch + 8)];
+            *dst = (add ? *dst : 0) + g;
+        }
+        __syncthreads();
+    };
+    bool full_used = false, part_used = false;  // D at column 0 / 128 holds products since the start or the last fold
+    auto drain = [&](bool add) {
+        if (full_used) {
+            drain_one(0, T, add);
+            add = true;
+        }
+        if (part_used) drain_one(128, rlast, add);
+    };
+
+    // thread i < 64 with (dy, dx) = (i / 8, i % 8) both < WIN sums S of that window sample, reference index dx * WIN + dy;
+    // thread 8 HALF + 7, the source row of the centre group, sums Sx.  No other thread reads the row sums.
+    const int  dy = tid >> 3, dx = tid & 7, pidx = dx * WIN + dy;
+    const bool wlane = dy < WIN && dx < WIN, slane = wlane || tid == 8 * HALF + 7;
+    long long  ssum = 0, npix = 0;
+    int        pending = 0;               // pixels in the s32 accumulators
+    bool       spilled = false;           // the partial already holds folded totals
+    uint32_t   inflight = 0, phase = 0;   // per buffer (bit b): MMAs committed and not yet waited for; barrier parity
+    auto wait_buf = [&](int b) {
+        if (inflight >> b & 1u) {
+            tc_bar_wait(&bar[b], phase >> b & 1u);
+            phase ^= 1u << b;
+            inflight &= ~(1u << b);
+        }
+    };
+    for (int tl = part, j = 0; tl < ntiles; tl += parts, j++) {
+        const int b  = j & 1;
+        const int ty = tl / ntx, tx = tl - ty * ntx;
+        const int r0 = s.v_start + ty * TH, c0 = s.h_start + tx * kTcTW;
+        const int nrows = min(TH, s.v_end - r0), ncols = min(kTcTW, s.h_end - c0);
+        __syncthreads();  // the zeroing of rsum[b] (previous tile) is done
+        if (pending + nrows * ncols > kTcFoldPixels) {  // CTA-uniform
+            wait_buf(b ^ 1);                            // the previous tile's MMAs and, with them, every earlier one
+            tc_fence_after();
+            drain(spilled);
+            tc_fence_before();
+            spilled   = true;
+            full_used = part_used = false;
+            pending   = 0;
+        }
+        wait_buf(b);  // the tensor core no longer reads this buffer
+        uint8_t* op = smem + b * kTcBufBytes;
+        int*     rs = rsum + b * kTcRowSums;
+        tc_build<WIN>(op, rs, dgd, src, s.dgd_stride, s.src_stride, r0, c0, nrows, ncols);
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // generic-proxy writes -> tensor-core reads
+        __syncthreads();
+        if (tid == 0) {
+            tc_fence_after();
+            const uint64_t d0 = tc_desc(tc_smem(op));
+            const int      nk = (ncols + 31) >> 5;
+            for (int y = 0; y < nrows; y += T) {
+                const bool full = y + T <= nrows;
+                bool&      used = full ? full_used : part_used;
+                for (int k = 0; k < nk; k++) {
+                    tc_mma_i8(tmem + (full ? 0u : 128u), d0 + (uint64_t)((y * kTcGrpBytes + k * 256) >> 4), IDESC, used ? 1u : 0u);
+                    used = true;
+                }
+            }
+            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(tc_smem(&bar[b])) : "memory");
+        } else {  // the same bookkeeping in every thread (CTA-uniform: drain() depends on it)
+            if (nrows >= T) full_used = true;
+            if (nrows % T) part_used = true;
+        }
+        inflight |= 1u << b;
+        if (slane) {  // S of this tile: the row sums of groups dy .. dy + nrows - 1, row dx
+            int t = 0;
+            for (int y = 0; y < nrows; y++) t += rs[(y + dy) * 8 + dx];
+            ssum += t;
+        }
+        __syncthreads();
+        for (int i = tid; i < kTcRowSums; i += kTcThreads) rs[i] = 0;
+        pending += nrows * ncols;
+        npix += nrows * ncols;
+    }
+    wait_buf(0);
+    wait_buf(1);
+    tc_fence_after();
+    drain(spilled);
+    if (wlane) P[kPartS + pidx] = ssum;
+    if (tid == 8 * HALF + 7) P[kPartSx] = ssum;
+    if (tid == 0) P[kPartN] = npix;
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) {
+        tc_fence_after();
+        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTcTmemCols) : "memory");
+    }
+}
+
+__global__ void __launch_bounds__(kTcThreads)
 stats_mma_kernel(const uint8_t* __restrict__ dgd_base, const uint8_t* __restrict__ src_base, const SvtB200StatsItem* __restrict__ items,
-                 const unsigned long long* __restrict__ tot_in, int ctas_per_item, long long* __restrict__ partial) {
-    __shared__ uint32_t tile[kMmaWords];
-    __shared__ int      s32[kMmaAccMax];
+                 int ctas_per_item, long long* __restrict__ partial) {
+    extern __shared__ __align__(1024) uint8_t smem[];
     const int it = blockIdx.x / ctas_per_item, part = blockIdx.x % ctas_per_item;
     const SvtB200StatsItem s = items[it];
-    const int avg = stats_average(tot_in, it, s);
-    if (part >= stats_mma_parts(s, ctas_per_item)) return;  // more CTAs than tiles: finalize ignores the unused partials
-    long long* P = partial + ((size_t)it * ctas_per_item + part) * 2450;
+    if (part >= stats_mma_parts(s, ctas_per_item)) return;  // more CTAs than tiles (before the TMEM allocation)
+    long long* P = partial + ((size_t)it * ctas_per_item + part) * kStatsPartWords;
     const uint8_t* dgd = dgd_base + s.dgd_off;
     const uint8_t* src = src_base + s.src_off;
-    if (s.wiener_win == 7) stats_mma_body<7>(dgd, src, s, avg, part, ctas_per_item, P, tile, s32);
-    else if (s.wiener_win == 5) stats_mma_body<5>(dgd, src, s, avg, part, ctas_per_item, P, tile, s32);
-    else stats_mma_body<3>(dgd, src, s, avg, part, ctas_per_item, P, tile, s32);
+    if (s.wiener_win == 7) stats_tc_body<7>(dgd, src, s, part, ctas_per_item, P, smem);
+    else if (s.wiener_win == 5) stats_tc_body<5>(dgd, src, s, part, ctas_per_item, P, smem);
+    else stats_tc_body<3>(dgd, src, s, part, ctas_per_item, P, smem);
 }
 
-// One thread per output element: it knows where its accumulator sits in a partial, adds that entry of
-// every part that was written, applies the bit-depth divider.  grid = (ceil(2450 / 256), n_items).
+// One thread per output element: adds its terms over every partial that was written and applies the mean expansion
+// above.  grid = (ceil(2450 / 256), n_items).
 __global__ void __launch_bounds__(256)
-stats_finalize_kernel(const long long* __restrict__ partial, int parts, const SvtB200StatsItem* __restrict__ items, int divider,
-                      int mma_layout, long long* __restrict__ M_out, long long* __restrict__ H_out) {
+stats_finalize_kernel(const long long* __restrict__ partial, int parts, const SvtB200StatsItem* __restrict__ items,
+                      long long* __restrict__ M_out, long long* __restrict__ H_out) {
     const int it = blockIdx.y, e = blockIdx.x * blockDim.x + threadIdx.x;
-    const int win = items[it].wiener_win, win2 = win * win;
-    if (e >= win2 * win2 + win2) return;
-    const int used = mma_layout ? stats_mma_parts(items[it], parts) : parts;
-    int       src;
-    if (e < win2 * win2) {
-        const int k = e / win2, l = e - k * win2;
-        int ka = k / win, kq = k - ka * win, la = l / win, lq = l - la * win;
-        if (mma_layout) {
-            // accumulator (row i = 8*kx+ky, column j) of the MMA lives in tile (i/16, j/8), C-fragment
-            // register ((i/8)&1)*2 + (j&1) of lane (i&7)*4 + (j&7)/2; only tiles with kx_i <= kx_j exist
-            if (ka > la) {
-                int x = ka; ka = la; la = x;
-                x = kq; kq = lq; lq = x;
-            }
-            src = (mma_tile_index(win, ka >> 1, la) * 4 + (ka & 1) * 2 + (lq & 1)) * 32 + kq * 4 + (lq >> 1);
-        } else {
-            // tiles were accumulated for window-column pairs a<=b only: element (k,l) lives in the
-            // tile of (k/win, l/win) when k/win <= l/win, else in its mirror
-            src = (ka <= la) ? k * win2 + l : l * win2 + k;
-        }
+    const int win = items[it].wiener_win, w2 = win * win;
+    if (e >= w2 * w2 + w2) return;
+    const int        used = stats_mma_parts(items[it], parts);
+    const long long* P    = partial + (size_t)it * parts * kStatsPartWords;
+    auto total = [&](int w) {
+        long long v = 0;
+        for (int p = 0; p < used; p++) v += P[(size_t)p * kStatsPartWords + w];
+        return v;
+    };
+    const long long n = total(kPartN), v = total(kPartS + w2 / 2) / n, nvv = n * v * v;
+    if (e < w2 * w2) {
+        const int k = e / w2, l = e - k * w2;
+        const long long g = total(kPartG + stats_tri_index(w2, min(k, l), max(k, l)));
+        H_out[(size_t)it * 2401 + e] = g - v * (total(kPartS + k) + total(kPartS + l)) + nvv;
     } else {
-        const int k = e - win2 * win2, ka = k / win, kq = k - ka * win;
-        src = mma_layout ? (mma_tile_index(win, 0, ka) * 4 + (kq & 1)) * 32 + 28 + (kq >> 1) : 2401 + k;  // M = matrix row 7
+        const int k = e - w2 * w2;
+        M_out[(size_t)it * 49 + k] = total(kPartGx + k) - v * (total(kPartS + k) + total(kPartSx)) + nvv;
     }
-    long long v = 0;
-    for (int p = 0; p < used; p++) v += partial[((size_t)it * parts + p) * 2450 + src];
-    if (e < win2 * win2) H_out[(size_t)it * 2401 + e] = v / divider;
-    else M_out[(size_t)it * 49 + (e - win2 * win2)] = v / divider;
 }
 
 // scratch of the batch call (per-CTA partials, pixel totals), one per stream: calls enqueued on
@@ -342,16 +445,30 @@ static void launch_lag_bulk(const PIX* d_dgd, const PIX* d_src, const SvtB200Sta
     B200_LAUNCH_CHECK();
 }
 
-template <typename PIX>
-static void launch_stats_mma(const PIX* d_dgd, const PIX* d_src, const SvtB200StatsItem* d_items, int n, int bd, long long* d_M,
-                             long long* d_H, long long* d_acc, unsigned long long* d_tot, cudaStream_t st);
+// 8-bit statistics: stats_mma_kernel writes a partial per CTA with pixel tiles, stats_finalize_kernel combines them
+static void launch_stats_mma(const uint8_t* d_dgd, const uint8_t* d_src, const SvtB200StatsItem* d_items, int n, long long* d_M,
+                             long long* d_H, long long* d_acc, cudaStream_t st) {
+    // CTAs per item: ~6 per SM over the batch (two are resident per SM; the kernel gives each of them a few pixel tiles)
+    int cpi = (ctx().sm_count * 6) / (n > 0 ? n : 1);
+    if (cpi < 1) cpi = 1;
+    if (cpi > kStatsMaxParts) cpi = kStatsMaxParts;
+    static int attr = -1;
+    if (attr != epoch()) {
+        B200_CUDA_CHECK(cudaFuncSetAttribute(stats_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTcSmem));
+        attr = epoch();
+    }
+    stats_mma_kernel<<<n * cpi, kTcThreads, kTcSmem, st>>>(d_dgd, d_src, d_items, cpi, d_acc);
+    B200_LAUNCH_CHECK();
+    stats_finalize_kernel<<<dim3((2450 + 255) / 256, n), 256, 0, st>>>(d_acc, cpi, d_items, d_M, d_H);
+    B200_LAUNCH_CHECK();
+}
 
 // Wiener statistics of a batch of units: 8-bit pictures on the tensor cores (stats_mma_kernel), 10 / 12 bit by lag sums
 // (wiener_stats_lag.cuh) -- both exact
 template <typename PIX>
 static void launch_stats(const PIX* d_dgd, const PIX* d_src, const SvtB200StatsItem* d_items, int n, int bd, long long* d_M,
                          long long* d_H, long long* d_acc, unsigned long long* d_tot, cudaStream_t st) {
-    if constexpr (sizeof(PIX) == 1) return launch_stats_mma<PIX>(d_dgd, d_src, d_items, n, bd, d_M, d_H, d_acc, d_tot, st);
+    if constexpr (sizeof(PIX) == 1) return launch_stats_mma(d_dgd, d_src, d_items, n, d_M, d_H, d_acc, st);
     const int divider = bd == 12 ? 16 : (bd == 10 ? 4 : 1);
     int cpi = (ctx().sm_count * 8) / (n > 0 ? n : 1);  // CTAs per unit: ~8 resident CTAs per SM over the batch
     if (cpi < 1) cpi = 1;
@@ -372,24 +489,6 @@ static void launch_stats(const PIX* d_dgd, const PIX* d_src, const SvtB200StatsI
 }
 
 template <typename PIX>
-static void launch_stats_mma(const PIX* d_dgd, const PIX* d_src, const SvtB200StatsItem* d_items, int n, int bd, long long* d_M,
-                             long long* d_H, long long* d_acc, unsigned long long* d_tot, cudaStream_t st) {
-    const int divider = bd == 12 ? 16 : (bd == 10 ? 4 : 1);
-    // CTAs per item: enough for ~6 resident CTAs per SM (the tensor-core kernel gives each of them 1-2 pixel tiles)
-    int cpi = (ctx().sm_count * (sizeof(PIX) == 1 ? 6 : 4)) / (n > 0 ? n : 1);
-    if (cpi < 1) cpi = 1;
-    if (cpi > (sizeof(PIX) == 1 ? kStatsMaxParts : 16)) cpi = sizeof(PIX) == 1 ? kStatsMaxParts : 16;
-    B200_CUDA_CHECK(cudaMemsetAsync(d_tot, 0, (size_t)n * sizeof(unsigned long long), st));
-    stats_sum_kernel<PIX><<<n * kSumParts, 256, 0, st>>>(d_dgd, d_items, d_tot);
-    B200_LAUNCH_CHECK();
-    static_assert(sizeof(PIX) == 1, "the tensor-core statistics are the 8-bit path (high bit depth: wiener_stats_lag.cuh)");
-    stats_mma_kernel<<<n * cpi, kMmaWarps * 32, 0, st>>>(d_dgd, d_src, d_items, d_tot, cpi, d_acc);
-    B200_LAUNCH_CHECK();
-    stats_finalize_kernel<<<dim3((2450 + 255) / 256, n), 256, 0, st>>>(d_acc, cpi, d_items, divider, sizeof(PIX) == 1, d_M, d_H);
-    B200_LAUNCH_CHECK();
-}
-
-template <typename PIX>
 static void stats_t1(int wiener_win, const PIX* dgd, const PIX* src, int h_start, int h_end, int v_start, int v_end, int dgd_stride,
                      int src_stride, int64_t* M, int64_t* H, int bd) {
     require_ready();
@@ -399,7 +498,7 @@ static void stats_t1(int wiener_win, const PIX* dgd, const PIX* src, int h_start
     LaneGuard l;
     size_t o_d = l->alloc((size_t)dw * dh * sizeof(PIX)), o_s = l->alloc((size_t)w * h * sizeof(PIX)), o_it = l->alloc(sizeof(SvtB200StatsItem));
     size_t in_end = l->used;
-    size_t o_M = l->alloc(49 * 8), o_H = l->alloc(2401 * 8), o_acc = l->alloc((size_t)kStatsMaxParts * 2450 * 8), o_avg = l->alloc(16);
+    size_t o_M = l->alloc(49 * 8), o_H = l->alloc(2401 * 8), o_acc = l->alloc(kStatsItemWords * 8), o_avg = l->alloc(16);
     for (int r = 0; r < dh; r++)
         memcpy(l->h<PIX>(o_d) + (size_t)r * dw, dgd + (ptrdiff_t)(v_start - half + r) * dgd_stride + h_start - half, dw * sizeof(PIX));
     for (int r = 0; r < h; r++) memcpy(l->h<PIX>(o_s) + (size_t)r * w, src + (ptrdiff_t)(v_start + r) * src_stride + h_start, w * sizeof(PIX));
@@ -498,7 +597,7 @@ extern "C" int svt_b200_compute_stats_batch_dev(const void* d_dgd, const void* d
     StatsScratch& sc = g_stats[(cudaStream_t)stream];
     if ((size_t)n_items > sc.cap) {
         sc.cap = (size_t)n_items * 2;  // new buffers; the old ones live on until shutdown (captured graphs may replay them)
-        sc.acc = (long long*)scratch_alloc(sc.cap * kStatsMaxParts * 2450 * 8);
+        sc.acc = (long long*)scratch_alloc(sc.cap * kStatsItemWords * 8);
         sc.tot = (unsigned long long*)scratch_alloc(sc.cap * 8);
     }
     if (bit_depth > 8)

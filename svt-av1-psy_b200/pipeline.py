@@ -339,7 +339,7 @@ class FramePipeline:
              ("cdef_apply", "cdef", "cdef_apply_kernel"),
              ("lr_boundaries", "rest", "lr_save_boundary_kernel x2"),
              ("rest_extend", "rest", "pad_plane_kernel"),
-             ("wiener_stats", "rest", "stats_sum_kernel+stats_mma_kernel+stats_finalize_kernel"),
+             ("wiener_stats", "rest", "stats_mma_kernel+stats_finalize_kernel (8-bit; 10-bit: stats_sum_kernel+stats_lag_*)"),
              ("wiener_filter", "rest", "lr_filter_kernel (striped restoration of the whole picture)"))
 
     def _stage(self, stage, s):
